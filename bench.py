@@ -51,7 +51,23 @@ def parse():
                     help="how many of them the CPU pipeline also runs (trajectory error and keyframe decisions)")
     ap.add_argument("--beams", type=int, default=64)
     ap.add_argument("--azimuths", type=int, default=2048)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed registration returned in its last step to DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
+    return a
+
+
+def dump_outputs(path, res):
+    """The arrays a caller of the timed registration receives (pose, last round's H and b, matched flags and their
+    count), one float64 / float32 .npy each.  The inputs are seeded, so the same arguments give the same inputs and two
+    builds can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    for name in ("X", "H", "b"):
+        np.save(os.path.join(path, f"{name}.npy"), np.asarray(res[name], dtype=np.float64))
+    np.save(os.path.join(path, "matched.npy"), np.asarray(res["matched"], dtype=np.float32))
+    np.save(os.path.join(path, "n_matched.npy"), np.array([res["n_matched"]], dtype=np.float64))
 
 
 def workload_name(a, n):
@@ -667,6 +683,8 @@ def main():
             line["sharded"] = sharded
         if stream:
             line["stream"] = stream
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, res)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()

@@ -1,9 +1,13 @@
-"""The CPU-runnable part of bench.py's contract: the reference arm prints one JSON line with the keys the
-driver reads, and without a GPU the product arm fails loudly instead of falling back."""
+"""bench.py's contract: the reference arm prints one JSON line with the keys a reader of the line expects, without a
+GPU the product arm fails loudly instead of falling back, and (`-m gpu`) --dump-outputs writes what the timed
+registration returned."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -41,6 +45,35 @@ def test_product_arm_needs_a_gpu(built):
     p = _run("--steps", "1", "--warmup", "1", "--beams", "8", "--azimuths", "256", "--no-cpu-baseline")
     assert p.returncode != 0
     assert "CUDA" in (p.stderr + p.stdout)
+
+
+def test_dump_outputs_is_for_the_product_arm(tmp_path):
+    p = _run("--impl", "reference", "--steps", "1", "--dump-outputs", str(tmp_path / "out"))
+    assert p.returncode == 2 and "--dump-outputs" in p.stderr
+    assert not (tmp_path / "out").exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_timed_registration(built, tmp_path):
+    """The last timed step's pose, H, b, matched flags and their count, as float64 / float32 .npy files; --steps sets
+    the number of timed steps; a second run with the same arguments computes the same arrays bit for bit."""
+    args = ("--steps", "3", "--warmup", "1", "--beams", "8", "--azimuths", "256", "--no-cpu-baseline", "--stream-scans", "0")
+    dumps = []
+    for run in ("a", "b"):
+        p = _run(*args, "--dump-outputs", str(tmp_path / run))
+        assert p.returncode == 0, p.stderr[-2000:]
+        line = json.loads(p.stdout.strip().splitlines()[-1])
+        assert line["steps"] == 3
+        d = {n: np.load(tmp_path / run / f"{n}.npy") for n in ("X", "H", "b", "matched", "n_matched")}
+        assert sorted(os.listdir(tmp_path / run)) == sorted(f"{n}.npy" for n in d)
+        assert d["X"].shape == (3, 4) and d["H"].shape == (6, 6) and d["b"].shape == (6,)
+        assert d["X"].dtype == d["H"].dtype == d["b"].dtype == np.float64 and d["matched"].dtype == np.float32
+        assert d["matched"].shape == (line["config"]["moving_leaves"],) and set(np.unique(d["matched"])) <= {0.0, 1.0}
+        assert d["n_matched"][0] == d["matched"].sum() == line["result"]["n_matched"]
+        assert d["X"][:, 3].tolist() == line["result"]["pose_t"]
+        dumps.append(d)
+    for n in dumps[0]:
+        assert np.array_equal(dumps[0][n], dumps[1][n]), n
 
 
 def test_ranks_next_to_one_socket_get_whole_physical_cores():

@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 
 from mad_icp_b200 import FlatTree, MadIcpError, Registrar, synth
-from util import HB_REL, POSE_M, POSE_RAD, bits_equal, pose_error
+from util import HB_REL, POSE_M, POSE_RAD, bits_equal, pose_error, same
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
@@ -192,32 +192,26 @@ def test_full_size_cfg3_indices_and_pose(full16, oracle):
 
 
 def test_full_size_cfg3_against_the_compiled_reference(full16):
-    """The same check with the reference's OWN sources on the CPU side (oracle/_ref: mad_tree.cpp and
-    mad_icp.cpp compiled against oracle/eigen_standin, shipped prebuilt; tests/test_reference_pin.py):
-    GPU correspondences == the reference's own at every round / keyframe / leaf, H/b at its poses, final pose."""
-    from oracle import reference as R
-    if not os.path.exists(R._SO):
-        pytest.skip("oracle/_ref not shipped (it is built where /root/reference exists)")
+    """The same check against what the reference's OWN sources computed on the CPU (mad_tree.cpp and mad_icp.cpp
+    compiled against oracle/eigen_standin, stored in golden/reference_full16.npz by golden/make_reference_golden.py;
+    tests/test_reference_pin.py): GPU correspondences == the reference's own at every round / keyframe / leaf, H/b at
+    its poses, final pose."""
     c, (reg, _, _) = full16
-    rtrees = []
-    for scan, P in zip(c["scans"], c["kf_poses"]):
-        t = R.ReferenceTree(scan, max_parallel_level=2)
-        t.apply_transform(P)
-        rtrees.append(t)
-    rq = R.ReferenceTree(c["query"])
-    ref = R.icp_run(rtrees, rq, c["T_guess"], iters=10, num_threads=min(16, R.max_threads()), record_idx=True)
+    with np.load(os.path.join(GOLD, "reference_full16.npz"), allow_pickle=False) as z:
+        ref = dict(z)
+    assert same(c["query"], ref["query.input"]) and all(same(s, ref[f"scan{k}.input"]) for k, s in enumerate(c["scans"]))
     # the reference's OWN correspondences (its bestMatchingLeafFast on its own X_ * mean_, mad_icp.cpp:78-79),
     # every round, every keyframe, every moving leaf: bit-exact, no sampling
     for it in range(10):
-        idx = reg.search(ref["X_hist"][it])
-        assert idx.shape == ref["idx_hist"][it].shape == (16, rq.num_leaves)
-        assert (idx == ref["idx_hist"][it]).all(), f"round {it}: {(idx != ref['idx_hist'][it]).sum()} differ"
-        H, b, _ = reg.linearize(ref["X_hist"][it])
-        _check_Hb(H, b, ref["H_hist"][it], ref["b_hist"][it], tol=10 * HB_REL)
+        idx = reg.search(ref["loop.X_hist"][it])
+        assert idx.shape == (16, int(ref["num_leaves"]))
+        assert same(idx, ref[f"loop.idx{it}"]), f"round {it}: correspondences differ from the reference's"
+        H, b, _ = reg.linearize(ref["loop.X_hist"][it])
+        _check_Hb(H, b, ref["loop.H_hist"][it], ref["loop.b_hist"][it], tol=10 * HB_REL)
     out = reg.register(c["T_guess"], iters=10)
-    ang, dt = pose_error(out["X"], ref["X"])
+    ang, dt = pose_error(out["X"], ref["loop.X"])
     assert ang < POSE_RAD and dt < POSE_M, (ang, dt)
-    assert (out["matched"] == ref["matched"]).mean() > 0.9999
+    assert (out["matched"] == ref["loop.matched"]).mean() > 0.9999
 
 
 def _moving_means(rtree):

@@ -1,109 +1,132 @@
 """Pins the CPU restatement (oracle/) against the reference's OWN sources.
 
-oracle/_ref/libmadicp_ref.so is tools/mad_tree.cpp, odometry/mad_icp.cpp, odometry/vel_estimator.cpp and
-odometry/pipeline.cpp compiled unmodified from /root/reference against oracle/eigen_standin (no Eigen in
-this image).  Everything the reference decides -- split order, leaf selection, normal inheritance, NaN
-handling of 1-point nodes, gate, kernel, accumulation order, keyframe promotion -- runs as written by its
-authors; the restatement must reproduce it bit for bit.  What stays unpinned is the evaluation order
-INSIDE Eigen's operators, which the stand-in takes from the restatement (see its header).
+tests/golden/reference_pin.npz holds what the reference computed -- tools/mad_tree.cpp, odometry/mad_icp.cpp,
+odometry/vel_estimator.cpp and odometry/pipeline.cpp compiled unmodified against oracle/eigen_standin
+(oracle/_ref/libmadicp_ref.so) -- on the inputs below; tests/golden/make_reference_golden.py wrote it.  Everything the
+reference decides -- split order, leaf selection, normal inheritance, NaN handling of 1-point nodes, gate, kernel,
+accumulation order, keyframe promotion -- runs as written by its authors; the restatement must reproduce it bit for
+bit.  What stays unpinned is the evaluation order INSIDE Eigen's operators, which the stand-in takes from the
+restatement (see its header).  Large arrays are stored as digests of their values (tests/util.py, fingerprint).
 
-CPU only.  Skipped where neither /root/reference nor a prebuilt oracle/_ref exists.
+CPU only.
 """
 import ctypes as C
+import os
 
 import numpy as np
 import pytest
 
 from mad_icp_b200 import synth
+from util import same
+
+GOLD = os.path.join(os.path.dirname(__file__), "golden", "reference_pin.npz")
+B_MAX_WALLS = (0.2, 1e-5)
+REG_CASES = ((1, 1), (3, 2), (4, 4))
+SWEEP = ((0.1, 0.05, 0.05, 0.01), (0.4, 0.2, 0.3, 0.05), (0.2, 0.1, 1e-3, 0.0))
+LOOP_KEYS = ("X_hist", "H_hist", "b_hist", "X", "matched")
 
 
-@pytest.fixture(scope="module")
-def ref(built):
-    from oracle import reference as R
-    if not R.available():
-        pytest.skip("no /root/reference and no prebuilt oracle/_ref")
-    R.lib()
-    return R
-
-
-def _same_tree(a, b):
-    ea, eb = a.export(), b.export()
-    assert a.num_nodes == b.num_nodes and a.num_leaves == b.num_leaves
-    for k in ea:
-        if ea[k].dtype.kind == "f":  # eigenvectors of 1-point nodes are NaN in both (0/0 covariance)
-            assert np.array_equal(ea[k], eb[k], equal_nan=True), k
-        else:
-            assert np.array_equal(ea[k], eb[k]), k
-    assert np.array_equal(a.cloud(), b.cloud())  # the build reorders and writes into the caller's vector
-
-
-@pytest.mark.parametrize("b_max", [0.2, 1e-5])
-def test_tree_build_is_the_references(oracle, ref, b_max):
+# ---- the inputs, shared with tests/golden/make_reference_golden.py
+def walls(points_per_wall):
     np.random.seed(42)
-    cloud = synth.four_walls(points_per_wall=2000)
-    _same_tree(oracle.OracleTree(cloud, b_max=b_max), ref.ReferenceTree(cloud, b_max=b_max))
+    return synth.four_walls(points_per_wall=points_per_wall)
+
+
+def degenerate_clouds():
+    rs = np.random.RandomState(3)
+    return (rs.rand(1, 3), rs.rand(2, 3), rs.rand(3, 3), np.repeat(rs.rand(1, 3), 50, axis=0),
+            np.c_[rs.rand(200, 2), np.zeros(200)], np.c_[rs.rand(64), np.zeros((64, 2))])
+
+
+def demo_guess():
+    """apps/utils/tools/mad_registration.py: the four-walls cloud (seed 42) and the initial guess drawn after it."""
+    cloud = walls(1000)
+    T = np.eye(4)
+    T[:3, :3] = synth.euler_xyz(0.1, 0.1, 0.1)
+    T[:3, 3] = np.random.rand(3)
+    return cloud, T
+
+
+def sequence(n, beams=16, azimuths=512):
+    scene = synth.StreetScene(seed=7)
+    for i in range(n):
+        base = synth.pose_xyyaw(0.8 * i, 1.0 + 0.02 * i, 0.004 * i)
+        yield 0.1 * i, np.ascontiguousarray(synth.lidar_scan(scene, base, beams=beams, azimuths=azimuths, seed=100 + i))
+
+
+DESKEW_POSES = (synth.pose_xyyaw(0.0, 1.0, 0.0), synth.pose_xyyaw(0.8, 1.05, 0.03))
+
+
+# ---- the checks
+@pytest.fixture(scope="module")
+def ref():
+    """The reference's results, by name."""
+    with np.load(GOLD, allow_pickle=False) as z:
+        return dict(z)
+
+
+def _same_tree(t, ref, key):
+    assert (t.num_nodes, t.num_leaves) == tuple(ref[f"{key}.size"]), key
+    for k, v in t.export().items():  # eigenvectors of 1-point nodes are NaN in both (0/0 covariance)
+        assert same(v, ref[f"{key}.{k}"]), (key, k)
+    assert same(t.cloud(), ref[f"{key}.cloud"]), key  # the build reorders and writes into the caller's vector
+
+
+def _same_loop(r, ref, key):
+    for k in LOOP_KEYS:
+        assert same(r[k], ref[f"{key}.{k}"]), (key, k)
+
+
+@pytest.mark.parametrize("b_max", B_MAX_WALLS)
+def test_tree_build_is_the_references(oracle, ref, b_max):
+    cloud = walls(2000)
+    assert same(cloud, ref[f"walls_{b_max}.input"])
+    _same_tree(oracle.OracleTree(cloud, b_max=b_max), ref, f"walls_{b_max}")
 
 
 def test_tree_build_lidar_scan_and_async_levels(oracle, ref):
     """max_parallel_level > 0 takes the reference's std::async branch (mad_tree.cpp:106-128): same tree."""
     case = synth.registration_case(K=1, beams=32, azimuths=1024)
     pts = case["scans"][0]
+    assert same(pts, ref["lidar.input"])
     o = oracle.OracleTree(pts)
-    _same_tree(o, ref.ReferenceTree(pts, max_parallel_level=0))
-    _same_tree(o, ref.ReferenceTree(pts, max_parallel_level=3))
+    _same_tree(o, ref, "lidar_level0")
+    _same_tree(o, ref, "lidar_level3")
     o.apply_transform(case["kf_poses"][0])
-    r = ref.ReferenceTree(pts)
-    r.apply_transform(case["kf_poses"][0])
-    _same_tree(o, r)
+    _same_tree(o, ref, "lidar_moved")
     q = case["query"][:5000]
-    assert np.array_equal(o.search(q), r.search(q))
+    assert same(o.search(q), ref["lidar_moved.search"])
 
 
 def test_degenerate_clouds(oracle, ref):
-    rs = np.random.RandomState(3)
-    for pts in (rs.rand(1, 3), rs.rand(2, 3), rs.rand(3, 3), np.repeat(rs.rand(1, 3), 50, axis=0),
-                np.c_[rs.rand(200, 2), np.zeros(200)], np.c_[rs.rand(64), np.zeros((64, 2))]):
-        _same_tree(oracle.OracleTree(pts, b_max=0.05), ref.ReferenceTree(pts, b_max=0.05))
+    for i, pts in enumerate(degenerate_clouds()):
+        _same_tree(oracle.OracleTree(pts, b_max=0.05), ref, f"degenerate{i}")
 
 
-@pytest.mark.parametrize("K,threads", [(1, 1), (3, 2), (4, 4)])
+@pytest.mark.parametrize("K,threads", REG_CASES)
 def test_registration_loop_is_the_references(oracle, ref, K, threads):
     case = synth.registration_case(K=K, beams=16, azimuths=512)
-    kfo, kfr = [], []
+    assert same(case["query"], ref[f"loop_{K}_{threads}.input"])
+    kfo = []
     for s in range(K):
-        a, b = oracle.OracleTree(case["scans"][s]), ref.ReferenceTree(case["scans"][s])
+        a = oracle.OracleTree(case["scans"][s])
         a.apply_transform(case["kf_poses"][s])
-        b.apply_transform(case["kf_poses"][s])
         kfo.append(a)
-        kfr.append(b)
-    mo, mr = oracle.OracleTree(case["query"]), ref.ReferenceTree(case["query"])
+    mo = oracle.OracleTree(case["query"])
     ro = oracle.icp_run(kfo, mo, case["T_guess"], iters=10, num_threads=threads)
-    rr = ref.icp_run(kfr, mr, case["T_guess"], iters=10, num_threads=threads, record_idx=True)
-    for k in ("X_hist", "H_hist", "b_hist", "X", "matched"):
-        assert np.array_equal(ro[k], rr[k]), k
+    _same_loop(ro, ref, f"loop_{K}_{threads}")
     # the correspondences themselves: the reference's bestMatchingLeafFast on its own X_ * mean_, every round
-    assert np.array_equal(np.asarray(ro["idx_hist"]), rr["idx_hist"])
+    for it in range(10):
+        assert same(np.asarray(ro["idx_hist"][it]), ref[f"loop_{K}_{threads}.idx{it}"]), it
 
 
 def test_four_walls_demo_is_the_references(oracle, ref):
     """apps/utils/tools/mad_registration.py through both: same 15 poses, same H/b, converge to identity."""
-    np.random.seed(42)
-    cloud = synth.four_walls(points_per_wall=1000)
-    T = np.eye(4)
-    T[:3, :3] = synth.euler_xyz(0.1, 0.1, 0.1)
-    T[:3, 3] = np.random.rand(3)
+    cloud, T = demo_guess()
+    assert same(cloud, ref["demo.input"]) and same(T, ref["demo.T"])
     ro = oracle.icp_run([oracle.OracleTree(cloud)], oracle.OracleTree(cloud), T, iters=15, record_matches=False)
-    rr = ref.icp_run([ref.ReferenceTree(cloud)], ref.ReferenceTree(cloud), T, iters=15)
-    for k in ("X_hist", "H_hist", "b_hist", "X", "matched"):
-        assert np.array_equal(ro[k], rr[k]), k
-    assert np.abs(rr["X"] - np.eye(4)[:3]).max() < 1e-6
-
-
-def _sequence(n, beams=16, azimuths=512):
-    scene = synth.StreetScene(seed=7)
-    for i in range(n):
-        base = synth.pose_xyyaw(0.8 * i, 1.0 + 0.02 * i, 0.004 * i)
-        yield 0.1 * i, np.ascontiguousarray(synth.lidar_scan(scene, base, beams=beams, azimuths=azimuths, seed=100 + i))
+    _same_loop(ro, ref, "demo")
+    assert np.abs(ref["demo.X"] - np.eye(4)[:3]).max() < 1e-6
 
 
 @pytest.mark.parametrize("deskew", [False, True])
@@ -119,19 +142,19 @@ def test_pipeline_is_the_references(oracle, ref, deskew):
     L.orc_pipeline_state.argtypes = [C.c_void_p, oracle._dp]
     L.orc_pipeline_free.argtypes = [C.c_void_p]
     po = C.c_void_p(L.orc_pipeline_create(10.0, int(deskew), 0.2, 0.1, 0.8, 0.1, 0.02, 4, 4, 0))
-    pr = ref.ReferencePipeline(deskew=deskew, num_keyframes=4, num_threads=4)
+    states = ref[f"pipeline_{deskew}.states"]
     st = np.zeros(23)
     promoted = 0
-    for i, (stamp, pts) in enumerate(_sequence(16)):
+    for i, (stamp, pts) in enumerate(sequence(16)):
+        assert same(pts, ref[f"sequence.input{i}"]), i
         L.orc_pipeline_compute(po, stamp, oracle._d(pts), pts.shape[0])
         L.orc_pipeline_state(po, oracle._d(st))
-        pr.compute(stamp, pts)
-        sr = pr.state()
+        sr = states[i]
         assert np.array_equal(st[:12], sr[:12]), i          # frame_to_map_
         assert np.array_equal(st[12:16], sr[12:16]), i      # map updated, ids, number of keyframes
         assert np.array_equal(st[17:], sr[17:]), i          # VelEstimator state
         promoted += int(st[12])
-    assert promoted >= 4
+    assert i == states.shape[0] - 1 and promoted >= 4
     L.orc_pipeline_free(po)
 
 
@@ -143,33 +166,28 @@ def test_deskew_is_the_references(oracle, ref):
     L.orc_pipeline_deskew.argtypes = [C.c_void_p, oracle._dp, C.c_int, oracle._dp, oracle._dp]
     L.orc_pipeline_free.argtypes = [C.c_void_p]
     po = C.c_void_p(L.orc_pipeline_create(10.0, 1, 0.2, 0.1, 0.8, 0.1, 0.02, 4, 1, 0))
-    pr = ref.ReferencePipeline(deskew=True, num_threads=1)
-    _, pts = next(_sequence(1))
-    Ta, Tb = synth.pose_xyyaw(0.0, 1.0, 0.0), synth.pose_xyyaw(0.8, 1.05, 0.03)
+    _, pts = next(sequence(1))
+    Ta, Tb = DESKEW_POSES
     mine = pts.copy()
     L.orc_pipeline_deskew(po, oracle._d(mine), mine.shape[0], oracle._d(np.ascontiguousarray(Ta[:3])),
                           oracle._d(np.ascontiguousarray(Tb[:3])))
-    assert np.array_equal(mine, pr.deskew(pts, Ta, Tb))
+    assert same(mine, ref["deskew.output"])
     assert np.abs(mine - pts).max() > 1e-3  # it did something
     L.orc_pipeline_free(po)
 
 
-@pytest.mark.parametrize("b_max,b_min,rho_ker,b_ratio", [(0.1, 0.05, 0.05, 0.01), (0.4, 0.2, 0.3, 0.05), (0.2, 0.1, 1e-3, 0.0)])
+@pytest.mark.parametrize("b_max,b_min,rho_ker,b_ratio", SWEEP)
 def test_parameter_sweep_is_the_references(oracle, ref, b_max, b_min, rho_ker, b_ratio):
     """Other leaf sizes, kernel widths and gate ratios than the defaults: trees and every GN round."""
     case = synth.registration_case(K=2, beams=16, azimuths=512, seed=9)
-    kfo, kfr = [], []
-    for s, P in zip(case["scans"], case["kf_poses"]):
-        a, b = oracle.OracleTree(s, b_max=b_max, b_min=b_min), ref.ReferenceTree(s, b_max=b_max, b_min=b_min)
-        _same_tree(a, b)
+    key = f"sweep_{b_max}_{b_min}_{rho_ker}_{b_ratio}"
+    kfo = []
+    for s, (scan, P) in enumerate(zip(case["scans"], case["kf_poses"])):
+        a = oracle.OracleTree(scan, b_max=b_max, b_min=b_min)
+        _same_tree(a, ref, f"{key}.kf{s}")
         a.apply_transform(P)
-        b.apply_transform(P)
         kfo.append(a)
-        kfr.append(b)
     mo = oracle.OracleTree(case["query"], b_max=b_max, b_min=b_min)
-    mr = ref.ReferenceTree(case["query"], b_max=b_max, b_min=b_min)
     ro = oracle.icp_run(kfo, mo, case["T_guess"], iters=6, min_ball=b_max, rho_ker=rho_ker, b_ratio=b_ratio, num_threads=2,
                         record_matches=False)
-    rr = ref.icp_run(kfr, mr, case["T_guess"], iters=6, min_ball=b_max, rho_ker=rho_ker, b_ratio=b_ratio, num_threads=2)
-    for k in ("X_hist", "H_hist", "b_hist", "X", "matched"):
-        assert np.array_equal(ro[k], rr[k], equal_nan=True) if ro[k].dtype.kind == "f" else np.array_equal(ro[k], rr[k]), k
+    _same_loop(ro, ref, key)

@@ -1,4 +1,38 @@
+import hashlib
+
 import numpy as np
+
+# arrays up to this size are stored whole in the golden files; larger ones as a digest
+GOLDEN_INLINE_BYTES = 16 << 10
+
+
+def digest(a):
+    """SHA-256 of an array's shape and values.  Integers hash as int64 and floats as float64 with every NaN made one NaN
+    and -0.0 made 0.0, so two arrays have the same digest exactly when np.array_equal(a, b, equal_nan=True) holds."""
+    a = np.asarray(a)
+    if a.dtype.kind == "f":
+        a = a.astype(np.float64)
+        a = np.where(np.isnan(a), np.nan, a + 0.0)
+    else:
+        a = a.astype(np.int64)
+    h = hashlib.sha256(repr(a.shape).encode())
+    h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
+def fingerprint(a):
+    """What a golden file keeps of an array: the array itself when it is small, its digest() otherwise."""
+    a = np.asarray(a)
+    return a.copy() if a.nbytes <= GOLDEN_INLINE_BYTES else np.str_(digest(a))
+
+
+def same(a, stored):
+    """Whether `a` is the array a golden file kept as `stored` (see fingerprint): np.array_equal, NaN equal to NaN."""
+    stored = np.asarray(stored)
+    if stored.dtype.kind == "U":
+        return digest(a) == str(stored)
+    a = np.asarray(a)
+    return a.shape == stored.shape and bool(np.array_equal(a, stored, equal_nan=a.dtype.kind == "f"))
 
 
 def bits_equal(a, b):
